@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the PCG hot path (BASELINE.json metric: PCG solves/sec + ms-to-tol per system; HBM roofline).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config c3|c5]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config c3|c5] [--dump-outputs DIR]
 
 Workload c3 (default; BASELINE config 3, config.workload): the TEST SET of 1024 independent 316x316 5-point
 variable-coefficient pressure systems (N = 99 856 unknowns each, the config-2 shape) with the factor L of a random-init
@@ -30,14 +30,21 @@ cpu_baseline / --impl reference: the CPU restatement of the reference loop (orac
           `A @` of cg.py:87), torch CPU CSR operands built on the CPU by oracle/sparse.py (the process never loads
           libdpcg.so), all host threads, on a bounded sample of the same workload. The reference itself is Python and
           cannot travel to the GPU box; tests pin the restatement to it.
+
+--dump-outputs DIR: after the timed steps, what the timed path returned in its last step, as DIR/<name>.npy (float64,
+          see dump_outputs). The workload is generated from fixed seeds, so two builds run with the same arguments can be
+          compared output for output.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 from pathlib import Path
@@ -70,9 +77,13 @@ def parse_args():
     ap.add_argument("--net", default="net", choices=["net", "tril"])
     ap.add_argument("--max-iter", type=int, default=MAX_ITER, help="profiling only: cap the bodies per solve")
     ap.add_argument("--no-extras", action="store_true", help="skip single-system latency and 128^3 kernel numbers")
+    ap.add_argument("--dump-outputs", type=Path, metavar="DIR",
+                    help="write what the timed path returned in its last step to DIR/<name>.npy")
     args = ap.parse_args()
     MAX_ITER = args.max_iter
     world = max(1, args.gpus)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.systems_total % args.step_systems or args.step_systems % world:
         ap.error("--systems-total must be a multiple of --step-systems, and --step-systems of --gpus")
     return args
@@ -112,6 +123,36 @@ def entry_bytes_of(batch):
         return 12
     mats = [m for e in batch.entries for m in [e["A"], *e["M"].stream_matrices()]]
     return 6 if all(m._packed for m in mats) else 12
+
+
+DUMP_X_BYTES = 48 << 20  # solutions and their positions; with the per-system arrays a dump stays under 64 MB
+
+
+def dump_outputs(directory, systems, results, systems_in_step, rank=0, world=1):
+    """--dump-outputs: the PcgResult of every system of the last timed step, as float64 arrays in `directory`:
+
+    systems.npy      index of each system in the workload
+    iterations.npy   PCG bodies run per system
+    res.npy          final value of the stopping criterion (squared relative residual) per system
+    x_hat.npy        solutions [system, position] at the positions of x_positions.npy (c5: in level order, the numbering
+                     the solve runs in)
+    x_positions.npy  every position when the solutions of a step fit DUMP_X_BYTES, else a sorted sample drawn by a
+                     generator with a fixed seed: the same for every run, system and rank (written by rank 0)
+
+    With several ranks, each rank writes its own systems as <name>.rank<r>.npy."""
+    directory.mkdir(parents=True, exist_ok=True)
+    n = results[0].x_hat.numel()
+    assert all(r.x_hat.numel() == n for r in results), "the systems of a step have one size"
+    k = min(n, DUMP_X_BYTES // (8 * (systems_in_step + 1)))
+    pos = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    index = torch.from_numpy(pos)
+    arrays = {"systems": systems, "iterations": [r.iterations for r in results], "res": [r.res for r in results],
+              "x_hat": torch.stack([r.x_hat[index.to(r.x_hat.device)].cpu() for r in results]).numpy()}
+    if rank == 0:
+        arrays["x_positions"] = pos
+    suffix = f".rank{rank}" if world > 1 else ""
+    for name, value in arrays.items():
+        np.save(directory / f"{name}{suffix}.npy", np.asarray(value, dtype=np.float64))
 
 
 # ---- clocks ------------------------------------------------------------------------------------------------------------
@@ -313,6 +354,8 @@ def run_reference(args):
         dt = time.perf_counter() - t0
         if step >= args.warmup:
             times.append(dt), iters.append(r.iterations)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [index], [r], 1)
     total = float(np.sum(times))
     value = len(times) / total
     sample = (f"1 system of the {args.systems_total}-system set per step ({len(times)} timed, distinct systems), cg.py:70-88 "
@@ -356,6 +399,8 @@ def run_reference_c5(args, threads):
         r = pcg.preconditioned_conjugate_gradient(a, b.clone(), m, rtol=RTOL, max_iter=sample_iters, as_is=True)
         if step >= args.warmup:
             times.append(r.seconds)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [0], [r], 1)
     per_iter = float(np.mean(times)) / sample_iters
     need = int(c5_iterations_hint().get(str(args.c5_side), 0)) or None
     value = 1.0 / (per_iter * need) if need else None
@@ -712,11 +757,16 @@ def extras(device, host0):
 
 
 def run_ours(args):
+    from deeppreconditioning_b200 import _lib
     from deeppreconditioning_b200 import build as dp_build
 
     rank, world, local = dist_setup(args)
-    if rank == 0:
-        dp_build.build()
+    if not os.environ.get("DPCG_LIB") and dp_build.stale():
+        # sources newer than the library in the tree: this process builds its own copy, outside the tree (which may be
+        # read-only)
+        tmp = Path(tempfile.mkdtemp(prefix="dpcg-"))
+        atexit.register(shutil.rmtree, tmp, True)
+        _lib.LIB_PATH = dp_build.build(force=True, out=tmp / "libdpcg.so")
     barrier(world)
     device = torch.device("cuda", local)
     if args.config == "c5":
@@ -784,6 +834,9 @@ def run_c3(args, rank, world, device):
     # results of every chunk that was solved (warm-up or timed): iteration statistics of the set
     solved = sorted({s % nchunks for s in range(nsteps)})
     results = {c: batches[c].results() for c in solved}
+    if args.dump_outputs:
+        last = (nsteps - 1) % nchunks
+        dump_outputs(args.dump_outputs, chunk_idx[last], results[last], args.step_systems, rank, world)
     kernel_ms = [k0.elapsed_time(k1) for _, k0, k1 in launches]
     entry_bytes = {c: entry_bytes_of(batches[c]) for c in solved}
     chunk_bytes = {c: sum(iter_bytes(e["A"].n, e["A"].nnz, e["M"].L.nnz, entry_bytes[c]) * r.iterations
@@ -952,6 +1005,8 @@ def run_c5(args, rank, world, device):
     local_ms = start.elapsed_time(stop)
     clocks = sampler.stop() if rank == 0 else None
     results = batch.results()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, mine, results, per_gpu * world, rank, world)
     its = [r.iterations for r in results]
     value = per_gpu * world * args.steps / (elapsed_ms / 1e3)
     local_bytes = float(sum(iter_bytes(n, nnz_a, nnz_l) * i for i in its))

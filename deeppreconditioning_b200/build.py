@@ -39,17 +39,19 @@ def stale() -> bool:
     return any(d.stat().st_mtime > t for d in deps)
 
 
-def build(force: bool = False, verbose: bool = False) -> Path:
+def build(force: bool = False, verbose: bool = False, out: Path = LIB) -> Path:
+    """Compile libdpcg.so to ``out`` (default: ``lib/libdpcg.so`` in the package). Without ``force`` nothing is compiled
+    while that default library is newer than its sources."""
     if not force and not stale():
         return LIB
-    LIB_DIR.mkdir(exist_ok=True)
-    cmd = [nvcc(), *NVCC_FLAGS, *(["-Xptxas", "-v"] if verbose else []), "-o", str(LIB), *[str(CSRC / s) for s in SOURCES]]
+    out.parent.mkdir(parents=True, exist_ok=True)
+    cmd = [nvcc(), *NVCC_FLAGS, *(["-Xptxas", "-v"] if verbose else []), "-o", str(out), *[str(CSRC / s) for s in SOURCES]]
     proc = subprocess.run(cmd, capture_output=True, text=True)
     if verbose or proc.returncode:
         sys.stderr.write(proc.stdout + proc.stderr)
     if proc.returncode:
         raise RuntimeError("nvcc failed building libdpcg.so")
-    return LIB
+    return out
 
 
 def build_variant(tag: str, defines: dict[str, int]) -> Path:

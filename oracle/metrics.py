@@ -1,9 +1,10 @@
 """ORACLE — dense restatement of ``uibk/deep_preconditioning/metrics.py`` (test infrastructure), on plain tensors.
 
 Inputs are the dense batches the reference gets from ``.dense()[:, 0]``: ``lower [B,N,N]`` (the CNN output ``L``) and
-``tril [B,N,N]`` (the stored lower triangle of ``A``). Pinned to the reference module itself where it can be imported
-(``tests/test_oracle.py::test_metrics_oracle_is_the_reference``): it only needs ``SparseConvTensor`` objects with
-``dense()`` / ``replace_feature``, which the stand-in in ``deeppreconditioning_b200.model`` provides.
+``tril [B,N,N]`` (the stored lower triangle of ``A``). Pinned to the values the reference module produced
+(``tests/golden/metrics_golden.json``, ``tests/test_oracle.py::test_metrics_oracle_matches_golden``): the reference
+only needs ``SparseConvTensor`` objects with ``dense()`` / ``replace_feature``, which the stand-in in
+``deeppreconditioning_b200.model`` provides.
 """
 
 from __future__ import annotations

@@ -299,3 +299,31 @@ def test_bench_line_helpers():
     n, nnz_a, nnz_l = 99856, 498016, 1494660
     assert bench.iter_bytes(n, nnz_a, nnz_l) == 12 * nnz_a + 24 * nnz_l + 132 * n + 12
     assert bench.iter_bytes(n, nnz_a, nnz_l) - bench.iter_bytes(n, nnz_a, nnz_l, 6) == 6 * (nnz_a + 2 * nnz_l)
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: float64 arrays of the last step's results, solutions sampled at positions that do not
+    change from run to run once a step's solutions exceed the budget, and the whole dump under 64 MB."""
+    import sys
+
+    sys.path.insert(0, str(ROOT))
+    import bench
+
+    gen = torch.Generator().manual_seed(0)
+    results = [PcgResult(0.0, 10 + i, 0, torch.randn(20000, dtype=torch.float64, generator=gen), 1e-9 * i) for i in range(3)]
+    for run in ("a", "b"):
+        bench.dump_outputs(tmp_path / run, [7, 9, 11], results, 4096)  # as if the step had 4096 systems: sampled
+    got = {f.name: np.load(f) for f in (tmp_path / "a").iterdir()}
+    assert set(got) == {"systems.npy", "iterations.npy", "res.npy", "x_hat.npy", "x_positions.npy"}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert all(np.array_equal(a, np.load(tmp_path / "b" / name)) for name, a in got.items())
+    pos = got["x_positions.npy"].astype(np.int64)
+    assert 0 < len(pos) < 20000 and np.all(np.diff(pos) > 0) and pos[-1] < 20000
+    assert np.array_equal(got["x_hat.npy"], np.stack([r.x_hat.numpy()[pos] for r in results]))
+    assert got["systems.npy"].tolist() == [7, 9, 11] and got["iterations.npy"].tolist() == [10, 11, 12]
+    assert got["res.npy"].tolist() == [r.res for r in results]
+    bench.dump_outputs(tmp_path / "c", [0], results[:1], 1)  # fits: every position
+    assert np.array_equal(np.load(tmp_path / "c" / "x_hat.npy")[0], results[0].x_hat.numpy())
+    x = torch.randn(99856, dtype=torch.float64, generator=gen)  # the default c3 step: 128 systems of 99 856 unknowns
+    bench.dump_outputs(tmp_path / "d", list(range(128)), [PcgResult(0.0, 1, 0, x, 0.0)] * 128, 128)
+    assert sum(f.stat().st_size for f in (tmp_path / "d").iterdir()) <= 64 << 20
