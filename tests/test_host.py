@@ -327,3 +327,16 @@ def test_bench_dump_outputs(tmp_path):
     x = torch.randn(99856, dtype=torch.float64, generator=gen)  # the default c3 step: 128 systems of 99 856 unknowns
     bench.dump_outputs(tmp_path / "d", list(range(128)), [PcgResult(0.0, 1, 0, x, 0.0)] * 128, 128)
     assert sum(f.stat().st_size for f in (tmp_path / "d").iterdir()) <= 64 << 20
+
+
+def test_schedule_model_mirrors_the_kernel_constants():
+    """The host-side model of the fused schedule in test_gpu_batch_scale.py (whose bite guards assert that its batches
+    reach several table rounds) uses the tile-table size and tile height the library is built with."""
+    from test_gpu_batch_scale import ROUND_TILES, TILE_ROWS
+
+    csrc = ROOT / "deeppreconditioning_b200" / "csrc"
+    defines = re.findall(r"^#define DPCG_ROUND_TILES (\d+)\s*$", (csrc / "pcg.cu").read_text(), re.M)
+    assert defines == [str(ROUND_TILES)], defines
+    assert not any("DPCG_ROUND_TILES" in flag for flag in build.NVCC_FLAGS), build.NVCC_FLAGS
+    common = (csrc / "common.cuh").read_text()
+    assert re.search(r"constexpr int kTileRows = kBlock;", common) and re.search(rf"constexpr int kBlock = {TILE_ROWS};", common)
