@@ -62,6 +62,13 @@ class PcgParams(C.Structure):
     _fields_ = [("rtol", C.c_double), ("max_iter", _i32), ("engine", _i32), ("check_every", _i32), ("reserved", _i32)]
 
 
+class SpconvLayer(C.Structure):
+    """``dp_spconv_layer_t``."""
+
+    _fields_ = [("nout", _i64), ("ntaps", _i32), ("cin", _i32), ("cout", _i32), ("reserved", _i32)] + [
+        (name, _p) for name in ("src", "in_", "weight", "bias", "slope", "head_weight", "head_bias", "indices", "out")]
+
+
 class DpcgError(RuntimeError):
     pass
 
@@ -106,6 +113,12 @@ _SIGNATURES = {
     "dp_sptrsv_ts_solve_batch_f64": (C.c_int, [C.POINTER(TrsvLsSystem), _i32, _p, _p, C.c_size_t, _p]),
     "dp_ic0_f64": (C.c_int, [_i32, _p, _p, _p, _p, _p, _i64, _i32, _p, _p, C.c_size_t, _p]),
     "dp_icholt_host": (C.c_int, [_i32, _p, _p, _p, _i32, C.c_double, _p, _p, _p, _i64, _p]),
+    "dp_spconv_sort_workspace_bytes": (C.c_size_t, [_i32, _i32]),
+    "dp_spconv_sort_sites": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _p, _p, _p, C.c_size_t, _p]),
+    "dp_spconv_rules_workspace_bytes": (C.c_size_t, [_i32, _i32, _i32]),
+    "dp_spconv_rules_count": (C.c_int, [_p, _p, _i32, _i32, _i32, _i32, _i32, _p, _p, C.c_size_t, _p]),
+    "dp_spconv_rules_fill": (C.c_int, [_p, _p, _p, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p]),
+    "dp_spconv_layer_f32": (C.c_int, [C.POINTER(SpconvLayer), _p]),
     "dp_pcg_work_doubles": (_i64, [_i32]),
     "dp_pcg_workspace_bytes": (C.c_size_t, [_i32]),
     "dp_debug_pcg_trace": (C.c_int, [_p, _i32, _p, _i32]),

@@ -172,3 +172,110 @@ class PreconditionerTrilNet(nn.Module):
 
 
 DEFAULT_CHANNELS = [1, 16, 32, 64, 32, 16, 1]  # params.yaml:6-13
+
+
+class InferenceNet:
+    """Inference-only forward of a :class:`PreconditionerNet` or :class:`PreconditionerTrilNet` on ``libdpcg``'s sparse
+    convolution kernels (``dp_spconv_*``, sm_100a): site sort, per-row rule merge of the 2x2 layers, one gather-GEMM
+    launch per layer with bias and activation in its epilogue, and the final 1x1 layer and output tail fused into the
+    layer before it.
+
+    The module's contract: ``SparseConvTensor -> SparseConvTensor`` for any ``batch_size``, same ``indices`` (sorted by
+    (batch, row, col) after a 2x2 layer, the input's own order for an all-1x1 network), ``spatial_shape`` and
+    ``batch_size`` as ``net(input)``, features fp32 ``[nnz, 1]``. CUDA tensors only, no autograd. The values are the fp32
+    forward in a fixed summation order (one fma chain per tap, taps added in (ky, kx) order, bias last), so they do not
+    depend on the batch a system is in. The parameters are read at every call: a later ``load_state_dict`` applies.
+    Usable wherever the module is called, e.g. ``BenchmarkSuite(data_set, InferenceNet(net))``.
+
+    Supported (checked here, without a GPU; anything else raises ``ValueError``): layers ``SparseConv2d`` with
+    ``kernel_size`` 1 (no padding) or 2 (padding ``(1, 0)`` or ``(0, 1)``) and 1..64 channels, each but the last
+    followed by at most one scalar ``PReLU`` / ``LeakyReLU``, the last with one output channel.
+    """
+
+    def __init__(self, net: nn.Module) -> None:
+        if not isinstance(net, (PreconditionerNet, PreconditionerTrilNet)):
+            raise ValueError(f"InferenceNet runs PreconditionerNet or PreconditionerTrilNet, not {type(net).__name__}")
+        steps: list[list] = []
+        for layer in net.layers:
+            if isinstance(layer, SparseConv2d):
+                _check_conv(layer)
+                if steps and steps[-1][0].weight.shape[0] != layer.weight.shape[3]:
+                    raise ValueError("consecutive layers disagree on the channel count")
+                steps.append([layer, None])
+            elif isinstance(layer, (PReLU, LeakyReLU)):
+                if not steps or steps[-1][1] is not None:
+                    raise ValueError("an activation must follow a convolution")
+                if isinstance(layer, PReLU) and layer.weight.numel() != 1:
+                    raise ValueError("only a scalar PReLU (num_parameters=1) is supported")
+                steps[-1][1] = layer
+            else:
+                raise ValueError(f"unsupported layer {type(layer).__name__}")
+        if not steps or steps[-1][1] is not None or steps[-1][0].weight.shape[0] != 1:
+            raise ValueError("the network must end with a convolution to one channel")
+        self.net = net
+        self.steps = [tuple(s) for s in steps]
+        self._slopes: dict = {}
+
+    def _slope(self, act, device) -> torch.Tensor | None:
+        if act is None:
+            return None
+        if isinstance(act, PReLU):
+            return act.weight
+        key = (float(act.negative_slope), device)
+        if key not in self._slopes:
+            self._slopes[key] = torch.tensor([key[0]], dtype=torch.float32, device=device)
+        return self._slopes[key]
+
+    def __call__(self, input_: SparseConvTensor) -> SparseConvTensor:
+        from . import _lib, spconv
+
+        feats, indices = input_.features, input_.indices
+        if not (feats.is_cuda and indices.is_cuda):
+            raise _lib.DpcgError("InferenceNet runs on CUDA tensors only (no CPU fallback)")
+        if feats.dtype != torch.float32 or feats.dim() != 2 or feats.shape[1] != self.steps[0][0].weight.shape[3]:
+            raise _lib.DpcgError(f"InferenceNet needs fp32 features [nnz, {self.steps[0][0].weight.shape[3]}]")
+        device = feats.device
+        for conv, act in self.steps:
+            for p in [conv.weight, conv.bias] + ([act.weight] if isinstance(act, PReLU) else []):
+                if p is not None and p.device != device:
+                    raise _lib.DpcgError("InferenceNet: the network's parameters are not on the input's device")
+        batch, (h, w) = input_.batch_size, input_.spatial_shape
+        # patterns first (their sizes are read back once per 2x2 layer), then the layers back to back
+        rules: dict[int, torch.Tensor] = {}
+        out_indices = indices
+        last_k2 = max((i for i, (conv, _) in enumerate(self.steps) if conv.k == 2), default=None)
+        if last_k2 is not None:
+            rowptr, col, perm = spconv.sort_sites(indices, batch, h, w)
+            for i, (conv, _) in enumerate(self.steps):
+                if conv.k == 2:
+                    rowptr, col, rules[i], ind = spconv.conv_rules(rowptr, col, batch, h, w, conv.padding, perm,
+                                                                   with_indices=i == last_k2)
+                    perm = None  # later layers read features in sorted site order
+                    if ind is not None:
+                        out_indices = ind
+                h, w = h + 2 * conv.padding[0] - conv.k + 1, w + 2 * conv.padding[1] - conv.k + 1
+        steps = self.steps
+        head = None
+        if len(steps) > 1 and steps[-1][0].k == 1:
+            head, steps = steps[-1][0], steps[:-1]
+        x = feats
+        for i, (conv, act) in enumerate(steps):
+            last = i == len(steps) - 1
+            nout = int(rules[i].shape[0]) if i in rules else int(x.shape[0])
+            x = spconv.conv_layer(x, conv.weight, conv.bias, rules.get(i), nout, self._slope(act, device),
+                                  head.weight if (last and head is not None) else None,
+                                  head.bias if (last and head is not None) else None,
+                                  out_indices if last else None)
+        return SparseConvTensor(x, out_indices, [h, w], batch)
+
+
+def _check_conv(conv: SparseConv2d) -> None:
+    cout, k, _, cin = conv.weight.shape
+    if conv.k not in (1, 2):
+        raise ValueError(f"kernel_size {conv.k} is not supported (1 or 2)")
+    if conv.k == 1 and tuple(conv.padding) != (0, 0):
+        raise ValueError("a 1x1 layer must not pad")
+    if conv.k == 2 and tuple(conv.padding) not in ((1, 0), (0, 1)):
+        raise ValueError(f"padding {tuple(conv.padding)} of a 2x2 layer is not supported ((1, 0) or (0, 1))")
+    if not (1 <= cin <= 64 and 1 <= cout <= 64):
+        raise ValueError(f"{cin} -> {cout} channels: at most 64 are supported")

@@ -334,6 +334,56 @@ size_t dp_pcg_workspace_bytes(int32_t nsys);
 int dp_pcg_solve_f64(const dp_pcg_system_t* systems_host, int32_t nsys, const dp_pcg_params_t* params_host,
                      int32_t* flag_out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- K6: sparse-convolution inference of the factor network (model.PreconditionerNet / PreconditionerTrilNet) --------
+ * Replaces the generic PyTorch forward of model.SparseConv2d (key sets, torch.unique, one GEMM and one index_add_ per
+ * tap) for inference: stride 1, k = 1 or k = 2 with padding (1,0) / (0,1), at most 64 channels, scalar activations.
+ *
+ * Site sort: indices int32[nnz,3] = (batch,row,col) of an H x W image, unordered. rowptr int32[batch_size*h + 1] is the
+ * "site CSR" over the (batch,row) pairs, col int32[nnz] the columns sorted in each row, perm int32[nnz] the input
+ * position of each sorted site. Every site counts, zero-valued ones included. *flag_out (device int32) receives
+ * DP_ERR_STRUCTURE for a repeated site or one outside [0,batch_size) x [0,h) x [0,w) (such sites are left out). */
+size_t dp_spconv_sort_workspace_bytes(int32_t batch_size, int32_t h);
+int dp_spconv_sort_sites(const int32_t* indices, int64_t nnz, int32_t batch_size, int32_t h, int32_t w, int32_t* rowptr,
+                         int32_t* col, int32_t* perm, int32_t* flag_out, void* workspace, size_t workspace_bytes,
+                         void* stream);
+/* Rules of a 2x2 layer with padding (ph,pw) in {(1,0),(0,1)} on a sorted site CSR of an h x w image: output image
+ * ho = h + 2ph - 1 by wo = w + 2pw - 1; output site (y,x) is active iff an input site (y + ky - ph, x + kx - pw) is.
+ * Two steps, because the caller sizes the outputs: _count writes rowptr_out int32[batch_size*ho + 1] (the total at
+ * rowptr_out[batch_size*ho]); _fill writes col_out int32[nout] (sorted per row), rules int32[nout,4] (16-byte aligned):
+ * rules[s,2ky+kx] = the input site of tap (ky,kx), -1 where inactive, numbered as the sorted sites, or through perm
+ * (perm != NULL) in the numbering of the sorted sites' source. indices_out (optional) int32[nout,3] = (batch,row,col),
+ * the order torch.unique gives model.SparseConv2d. */
+size_t dp_spconv_rules_workspace_bytes(int32_t batch_size, int32_t h, int32_t ph);
+int dp_spconv_rules_count(const int32_t* rowptr_in, const int32_t* col_in, int32_t batch_size, int32_t h, int32_t w,
+                          int32_t ph, int32_t pw, int32_t* rowptr_out, void* workspace, size_t workspace_bytes,
+                          void* stream);
+int dp_spconv_rules_fill(const int32_t* rowptr_in, const int32_t* col_in, const int32_t* perm, int32_t batch_size,
+                         int32_t h, int32_t w, int32_t ph, int32_t pw, const int32_t* rowptr_out, int32_t* col_out,
+                         int32_t* rules, int32_t* indices_out, void* stream);
+/* One layer, fp32 on CUDA cores: out[s,co] = act(((0 + p_0) + p_1 ...) + bias[co]) with p_t = sum over ci ascending of
+ * weight[co,t,ci] * in[src[s,t],ci] (one fma chain per tap, inactive taps skipped), act(v) = v > 0 ? v : slope * v.
+ * The order is fixed per output value: results do not depend on the batch or the launch geometry.
+ * head_weight != NULL: the final 1x1 layer (cout -> 1) follows in the epilogue, y = sum_co head_weight[co] * out[s,co]
+ * (+ head_bias), and out is [nout,1]. indices != NULL: the output tail of the factor network on that one channel (the
+ * layer's own when cout == 1 without a head): sites with row < col are multiplied by 0, diagonal sites get softplus
+ * (threshold 20, log1p(exp(y))). All pointers are device pointers; weights are read at every call. */
+typedef struct dp_spconv_layer {
+    int64_t nout;              /* output sites */
+    int32_t ntaps;             /* 1 (k = 1) or 4 (k = 2, taps in (ky,kx) order) */
+    int32_t cin, cout;         /* 1..64 */
+    int32_t reserved;
+    const int32_t* src;        /* [nout, ntaps] input site per tap (-1: inactive); NULL: site s reads row s (ntaps 1) */
+    const float* in;           /* [*, cin] */
+    const float* weight;       /* [cout, ntaps, cin]: spconv's [out, k, k, in] */
+    const float* bias;         /* [cout] or NULL */
+    const float* slope;        /* device scalar (PReLU weight, LeakyReLU slope) or NULL: no activation */
+    const float* head_weight;  /* [cout] or NULL */
+    const float* head_bias;    /* [1] or NULL */
+    const int32_t* indices;    /* [nout,3] (batch,row,col) of the output sites for the tail, or NULL */
+    float* out;                /* [nout, cout], [nout, 1] with a head */
+} dp_spconv_layer_t;
+int dp_spconv_layer_f32(const dp_spconv_layer_t* layer_host, void* stream);
+
 /* Diagnostics: with DPCG_TRACE=1 in the environment the fused engine records (label, clock64) pairs of CTA 0 into the
  * workspace; this copies up to `capacity` pairs to out_host[2*capacity] (label = 8*phase + point). Synchronous. */
 int dp_debug_pcg_trace(const void* workspace, int32_t nsys, int64_t* out_host, int32_t capacity);
