@@ -69,6 +69,14 @@ class SpconvLayer(C.Structure):
         (name, _p) for name in ("src", "in_", "weight", "bias", "slope", "head_weight", "head_bias", "indices", "out")]
 
 
+class SpconvGrad(C.Structure):
+    """``dp_spconv_grad_t``."""
+
+    _fields_ = [("nout", _i64), ("ntaps", _i32), ("cin", _i32), ("cout", _i32), ("reserved", _i32)] + [
+        (name, _p) for name in ("src", "in_", "grad_out", "pre", "slope", "tail_indices", "grad_pre", "grad_weight",
+                                "grad_bias", "grad_slope")]
+
+
 class DpcgError(RuntimeError):
     pass
 
@@ -119,6 +127,11 @@ _SIGNATURES = {
     "dp_spconv_rules_count": (C.c_int, [_p, _p, _i32, _i32, _i32, _i32, _i32, _p, _p, C.c_size_t, _p]),
     "dp_spconv_rules_fill": (C.c_int, [_p, _p, _p, _i32, _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p]),
     "dp_spconv_layer_f32": (C.c_int, [C.POINTER(SpconvLayer), _p]),
+    "dp_spconv_layer_train_f32": (C.c_int, [C.POINTER(SpconvLayer), _p, _p, _p, _p]),
+    "dp_spconv_rules_invert": (C.c_int, [_p, _i64, _i32, _i64, _p, _p, _p]),
+    "dp_spconv_wgrad_chunk_sites": (_i32, []),
+    "dp_spconv_wgrad_workspace_bytes": (C.c_size_t, [_i64, _i32, _i32, _i32]),
+    "dp_spconv_wgrad_f32": (C.c_int, [C.POINTER(SpconvGrad), _p, C.c_size_t, _p]),
     "dp_pcg_work_doubles": (_i64, [_i32]),
     "dp_pcg_workspace_bytes": (C.c_size_t, [_i32]),
     "dp_debug_pcg_trace": (C.c_int, [_p, _i32, _p, _i32]),

@@ -16,7 +16,8 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB_DIR = PKG / "lib"
 LIB = LIB_DIR / "libdpcg.so"
-SOURCES = ["spmv.cu", "scan.cu", "assembly.cu", "levels.cu", "sptrsv.cu", "pcg.cu", "icholt.cu", "sparseconv.cu"]
+SOURCES = ["spmv.cu", "scan.cu", "assembly.cu", "levels.cu", "sptrsv.cu", "pcg.cu", "icholt.cu", "sparseconv.cu",
+           "sparseconv_grad.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17", "--fmad=false",

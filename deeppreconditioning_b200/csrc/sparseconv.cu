@@ -13,6 +13,9 @@
 //   y    = act(acc + bias)                                        scalar PReLU / LeakyReLU slope
 // The last layer before the final 1x1 (cout -> 1) also applies that 1x1 and the output tail of the reference
 // (strict upper triangle multiplied by 0, softplus on the diagonal) in its epilogue.
+// The training forward (dp_spconv_layer_train_f32) is the same kernel with kTrain set: it also stores what the backward
+// (sparseconv_grad.cu) reads - acc + bias before the activation, and in the fused epilogue the activated rows the head
+// reads and the head's value before the tail. Its `out` is bitwise the inference launch's.
 #include <math.h>
 
 #include "common.cuh"
@@ -185,8 +188,16 @@ __device__ __forceinline__ float softplus_f32(float x) {  // torch.nn.functional
     return x > 20.0f ? x : log1pf(expf(x));
 }
 
-template <int COUTP>
-__global__ void __launch_bounds__(kConvThreads, 2) conv_gemm_kernel(dp_spconv_layer_t L) {
+// What a training forward keeps (kTrain): pre [nout, cout] when the layer has an activation; with a head, hidden
+// [nout, cout] (the activated rows) and head_pre [nout]; with a tail and no head, head_pre [nout] (the value before it).
+struct ConvKeep {
+    float* pre;
+    float* hidden;
+    float* head_pre;
+};
+
+template <int COUTP, bool kTrain>
+__global__ void __launch_bounds__(kConvThreads, 2) conv_gemm_kernel(dp_spconv_layer_t L, ConvKeep keep) {
     using S = ConvShape<COUTP>;
     constexpr int kTM = S::kTM, kTN = S::kTN, kM = S::kM, kNY = S::kNY;
     extern __shared__ __align__(16) float smem[];
@@ -282,6 +293,10 @@ __global__ void __launch_bounds__(kConvThreads, 2) conv_gemm_kernel(dp_spconv_la
             for (int i = 0; i < kTM; ++i) {
                 float v = acc[i][j];
                 if (L.bias) v = __fadd_rn(v, bj);
+                if constexpr (kTrain) {
+                    const long long site = base + ty + kNY * i;
+                    if (L.slope && site < L.nout && co < cout) keep.pre[site * cout + co] = v;
+                }
                 if (L.slope) v = v > 0.0f ? v : __fmul_rn(slope, v);
                 acc[i][j] = v;
             }
@@ -306,6 +321,16 @@ __global__ void __launch_bounds__(kConvThreads, 2) conv_gemm_kernel(dp_spconv_la
             for (int i = 0; i < kTM; ++i)
 #pragma unroll
                 for (int j = 0; j < kTN; ++j) hs[(ty + kNY * i) * (COUTP + 1) + tx * kTN + j] = acc[i][j];
+            if constexpr (kTrain) {
+#pragma unroll
+                for (int i = 0; i < kTM; ++i) {
+                    const long long site = base + ty + kNY * i;
+                    if (site >= L.nout) continue;
+#pragma unroll
+                    for (int j = 0; j < kTN; ++j)
+                        if (tx * kTN + j < cout) keep.hidden[site * cout + tx * kTN + j] = acc[i][j];
+                }
+            }
             __syncthreads();
         }
         for (int s = head ? tid : (tx == 0 ? ty : kM); s < kM; s += head ? kConvThreads : kM) {
@@ -318,6 +343,9 @@ __global__ void __launch_bounds__(kConvThreads, 2) conv_gemm_kernel(dp_spconv_la
                 if (L.head_bias) y = __fadd_rn(y, *L.head_bias);
             } else {
                 y = acc[0][0];  // cout == 1 (checked), kTM == 1, thread tx 0 holds the site
+            }
+            if constexpr (kTrain) {
+                if (keep.head_pre) keep.head_pre[site] = y;
             }
             if (L.indices) {
                 const int r = L.indices[3 * site + 1], c = L.indices[3 * site + 2];
@@ -336,17 +364,17 @@ static int grid_for_items(long long items, int threads) {
     return b < 1 ? 1 : (int)b;
 }
 
-template <int COUTP>
-static int launch_conv(const dp_spconv_layer_t& L, cudaStream_t s) {
+template <int COUTP, bool kTrain>
+static int launch_conv(const dp_spconv_layer_t& L, ConvKeep keep, cudaStream_t s) {
     using S = ConvShape<COUTP>;
     const size_t smem = conv_smem_bytes<COUTP>(L.ntaps, L.cin, L.head_weight != nullptr);
-    const void* fn = reinterpret_cast<const void*>(conv_gemm_kernel<COUTP>);
+    const void* fn = reinterpret_cast<const void*>(conv_gemm_kernel<COUTP, kTrain>);
     int st = allow_dynamic_smem(fn, smem);
     if (st != DP_OK) return st;
     const long long tiles = (L.nout + S::kM - 1) / S::kM;
     const long long cap = coop_grid(fn, kConvThreads, smem);  // resident CTAs (cached per device): the grid strides
     const int grid = (int)(tiles < cap ? tiles : cap);
-    conv_gemm_kernel<COUTP><<<grid, kConvThreads, smem, s>>>(L);
+    conv_gemm_kernel<COUTP, kTrain><<<grid, kConvThreads, smem, s>>>(L, keep);
     DP_LAUNCH_CHECK();
     return DP_OK;
 }
@@ -356,6 +384,25 @@ static size_t sort_ws_bytes(long long rows) {
 }
 
 static bool rows_ok(int nb, int h) { return nb >= 0 && h >= 0 && (long long)nb * h < 0x7fffffffLL; }
+
+static int layer_args(const dp_spconv_layer_t& L) {
+    if (L.nout < 0 || L.nout > 0x7fffffffLL || (L.ntaps != 1 && L.ntaps != 4)) return DP_ERR_INVALID;
+    if (L.cin < 1 || L.cin > kMaxChannels || L.cout < 1 || L.cout > kMaxChannels) return DP_ERR_INVALID;
+    if (L.ntaps == 4 && !L.src) return DP_ERR_INVALID;                // identity sources exist for 1x1 layers only
+    if (L.indices && !L.head_weight && L.cout != 1) return DP_ERR_INVALID;  // the tail acts on one channel
+    return DP_OK;
+}
+
+template <bool kTrain>
+static int launch_layer(const dp_spconv_layer_t& L, ConvKeep keep, cudaStream_t s) {
+    const int c = L.cout;
+    if (c <= 1 && !L.head_weight) return launch_conv<1, kTrain>(L, keep, s);
+    if (c <= 4) return launch_conv<4, kTrain>(L, keep, s);
+    if (c <= 8) return launch_conv<8, kTrain>(L, keep, s);
+    if (c <= 16) return launch_conv<16, kTrain>(L, keep, s);
+    if (c <= 32) return launch_conv<32, kTrain>(L, keep, s);
+    return launch_conv<64, kTrain>(L, keep, s);
+}
 
 }  // namespace dp
 
@@ -444,20 +491,25 @@ int dp_spconv_rules_fill(const int32_t* rowptr_in, const int32_t* col_in, const 
 int dp_spconv_layer_f32(const dp_spconv_layer_t* layer_host, void* stream) {
     if (!layer_host) return DP_ERR_INVALID;
     const dp_spconv_layer_t& L = *layer_host;
-    if (L.nout < 0 || L.nout > 0x7fffffffLL || (L.ntaps != 1 && L.ntaps != 4)) return DP_ERR_INVALID;
-    if (L.cin < 1 || L.cin > kMaxChannels || L.cout < 1 || L.cout > kMaxChannels) return DP_ERR_INVALID;
-    if (L.ntaps == 4 && !L.src) return DP_ERR_INVALID;                // identity sources exist for 1x1 layers only
-    if (L.indices && !L.head_weight && L.cout != 1) return DP_ERR_INVALID;  // the tail acts on one channel
+    int st = layer_args(L);
+    if (st != DP_OK) return st;
     if (L.nout == 0) return DP_OK;
     if (!L.in || !L.weight || !L.out) return DP_ERR_INVALID;
-    cudaStream_t s = (cudaStream_t)stream;
-    const int c = L.cout;
-    if (c <= 1 && !L.head_weight) return launch_conv<1>(L, s);
-    if (c <= 4) return launch_conv<4>(L, s);
-    if (c <= 8) return launch_conv<8>(L, s);
-    if (c <= 16) return launch_conv<16>(L, s);
-    if (c <= 32) return launch_conv<32>(L, s);
-    return launch_conv<64>(L, s);
+    return launch_layer<false>(L, ConvKeep{nullptr, nullptr, nullptr}, (cudaStream_t)stream);
+}
+
+int dp_spconv_layer_train_f32(const dp_spconv_layer_t* layer_host, float* pre, float* hidden, float* head_pre,
+                              void* stream) {
+    if (!layer_host) return DP_ERR_INVALID;
+    const dp_spconv_layer_t& L = *layer_host;
+    int st = layer_args(L);
+    if (st != DP_OK) return st;
+    const bool head = L.head_weight != nullptr;
+    if (L.nout == 0) return DP_OK;
+    if (!L.in || !L.weight || !L.out) return DP_ERR_INVALID;
+    if ((L.slope && !pre) || (head && (!hidden || !head_pre)) || (L.indices && !head_pre)) return DP_ERR_INVALID;
+    return launch_layer<true>(L, ConvKeep{pre, head ? hidden : nullptr, (head || L.indices) ? head_pre : nullptr},
+                              (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -20,6 +20,7 @@ from __future__ import annotations
 
 import torch
 from torch import nn
+from torch.autograd.function import once_differentiable
 
 
 class SparseConvTensor:
@@ -226,21 +227,29 @@ class InferenceNet:
             self._slopes[key] = torch.tensor([key[0]], dtype=torch.float32, device=device)
         return self._slopes[key]
 
-    def __call__(self, input_: SparseConvTensor) -> SparseConvTensor:
-        from . import _lib, spconv
+    def _check_input(self, input_: SparseConvTensor) -> torch.device:
+        from . import _lib
 
         feats, indices = input_.features, input_.indices
         if not (feats.is_cuda and indices.is_cuda):
-            raise _lib.DpcgError("InferenceNet runs on CUDA tensors only (no CPU fallback)")
+            raise _lib.DpcgError(f"{type(self).__name__} runs on CUDA tensors only (no CPU fallback)")
         if feats.dtype != torch.float32 or feats.dim() != 2 or feats.shape[1] != self.steps[0][0].weight.shape[3]:
-            raise _lib.DpcgError(f"InferenceNet needs fp32 features [nnz, {self.steps[0][0].weight.shape[3]}]")
+            raise _lib.DpcgError(f"{type(self).__name__} needs fp32 features [nnz, {self.steps[0][0].weight.shape[3]}]")
         device = feats.device
         for conv, act in self.steps:
             for p in [conv.weight, conv.bias] + ([act.weight] if isinstance(act, PReLU) else []):
                 if p is not None and p.device != device:
-                    raise _lib.DpcgError("InferenceNet: the network's parameters are not on the input's device")
+                    raise _lib.DpcgError(f"{type(self).__name__}: the network's parameters are not on the input's device")
+        return device
+
+    def _plan(self, input_: SparseConvTensor):
+        """The launches of a forward: ``(layers, out_indices, spatial_shape)``, ``layers`` a list of ``(conv, act, rules
+        or None, head or None)``: one launch each, the final 1x1 fused as ``head`` into the last. All patterns are built
+        here, before the first GEMM (their sizes are read back once per 2x2 layer)."""
+        from . import spconv
+
+        indices = input_.indices
         batch, (h, w) = input_.batch_size, input_.spatial_shape
-        # patterns first (their sizes are read back once per 2x2 layer), then the layers back to back
         rules: dict[int, torch.Tensor] = {}
         out_indices = indices
         last_k2 = max((i for i, (conv, _) in enumerate(self.steps) if conv.k == 2), default=None)
@@ -258,15 +267,121 @@ class InferenceNet:
         head = None
         if len(steps) > 1 and steps[-1][0].k == 1:
             head, steps = steps[-1][0], steps[:-1]
-        x = feats
-        for i, (conv, act) in enumerate(steps):
-            last = i == len(steps) - 1
-            nout = int(rules[i].shape[0]) if i in rules else int(x.shape[0])
-            x = spconv.conv_layer(x, conv.weight, conv.bias, rules.get(i), nout, self._slope(act, device),
-                                  head.weight if (last and head is not None) else None,
-                                  head.bias if (last and head is not None) else None,
+        layers = [(conv, act, rules.get(i), head if i == len(steps) - 1 else None) for i, (conv, act) in enumerate(steps)]
+        return layers, out_indices, [h, w]
+
+    def __call__(self, input_: SparseConvTensor) -> SparseConvTensor:
+        from . import spconv
+
+        device = self._check_input(input_)
+        layers, out_indices, shape = self._plan(input_)
+        x = input_.features
+        for i, (conv, act, src, head) in enumerate(layers):
+            last = i == len(layers) - 1
+            nout = int(src.shape[0]) if src is not None else int(x.shape[0])
+            x = spconv.conv_layer(x, conv.weight, conv.bias, src, nout, self._slope(act, device),
+                                  head.weight if head is not None else None, head.bias if head is not None else None,
                                   out_indices if last else None)
-        return SparseConvTensor(x, out_indices, [h, w], batch)
+        return SparseConvTensor(x, out_indices, shape, input_.batch_size)
+
+
+class TrainableNet(InferenceNet):
+    """:class:`InferenceNet` with a backward on the device kernels: training of the factor network without the PyTorch
+    layers.
+
+    When autograd is enabled and a parameter of ``net`` requires grad, the call runs a ``torch.autograd.Function``: the
+    training forward (``dp_spconv_layer_train_f32``, output bitwise :class:`InferenceNet`'s) keeps every layer's input,
+    its value before the activation, the fused head's input and value before the tail, and each 2x2 layer's inverse
+    rules; its backward walks the layers in reverse, one weight-gradient launch (``dp_spconv_wgrad_f32``) and one
+    input-gradient launch (the forward kernel on the transposed weights and inverse rules) per layer. Gradients go to
+    ``net``'s own parameters (conv weights, biases, PReLU weights), so ``loss.backward()`` accumulates into their
+    ``.grad`` and ``torch.optim.*(net.parameters())`` works unchanged. They are deterministic: the same bits on every
+    run, and a system's input gradient at every layer does not depend on its batch.
+
+    Otherwise (``torch.no_grad()``, or no parameter requires grad) the call is exactly :class:`InferenceNet`'s. Input
+    features that require grad raise ``ValueError``: the first layer's input gradient is not computed.
+    """
+
+    def _parameters(self) -> list:
+        params = []
+        for conv, act in self.steps:
+            params += [conv.weight] + ([conv.bias] if conv.bias is not None else [])
+            if isinstance(act, PReLU):
+                params.append(act.weight)
+        return params
+
+    def __call__(self, input_: SparseConvTensor) -> SparseConvTensor:
+        params = self._parameters()
+        if not (torch.is_grad_enabled() and any(p.requires_grad for p in params)):
+            return super().__call__(input_)
+        if input_.features.requires_grad:
+            raise ValueError("TrainableNet does not compute the gradient of its input features")
+        self._check_input(input_)
+        layers, out_indices, shape = self._plan(input_)
+        feats = _DeviceTraining.apply(self, layers, out_indices, input_.features, *params)
+        return SparseConvTensor(feats, out_indices, shape, input_.batch_size)
+
+
+class _DeviceTraining(torch.autograd.Function):
+    """Forward and backward of :class:`TrainableNet` (inputs after ``out_indices``: the features, then the parameters in
+    ``TrainableNet._parameters`` order)."""
+
+    @staticmethod
+    def forward(ctx, inet, layers, out_indices, feats, *params):
+        from . import spconv
+
+        device = feats.device
+        saved = []
+        x = feats
+        for i, (conv, act, src, head) in enumerate(layers):
+            last = i == len(layers) - 1
+            nout = int(src.shape[0]) if src is not None else int(x.shape[0])
+            out, pre, hidden, head_pre = spconv.layer_train(
+                x, conv.weight, conv.bias, src, nout, inet._slope(act, device),
+                head.weight if head is not None else None, head.bias if head is not None else None,
+                out_indices if last else None)
+            inv = spconv.invert_rules(src, x.shape[0]) if (src is not None and i > 0) else None
+            saved.append((x, pre, hidden, head_pre, inv))
+            x = out
+        ctx.inet, ctx.layers, ctx.out_indices, ctx.saved = inet, layers, out_indices, saved
+        ctx.param_ids = [id(p) for p in params]
+        ctx.param_dtypes = [p.dtype for p in params]
+        return x
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_features):
+        from . import spconv
+
+        inet, layers, out_indices = ctx.inet, ctx.layers, ctx.out_indices
+        device = grad_features.device
+        grads: dict[int, torch.Tensor] = {}
+        g = grad_features.to(torch.float32).contiguous()
+        for i in reversed(range(len(layers))):
+            conv, act, src, head = layers[i]
+            x, pre, hidden, head_pre, inv = ctx.saved[i]
+            tail = None
+            if head is not None:  # the fused final 1x1 and the tail: its gradients, then g at the hidden rows
+                g_u, grads[id(head.weight)], db, _ = spconv.wgrad(hidden, g, head.weight.shape, pre=head_pre,
+                                                                  tail_indices=out_indices)
+                if head.bias is not None:
+                    grads[id(head.bias)] = db
+                g = spconv.conv_layer(g_u, head.weight.detach().permute(3, 1, 2, 0), None)
+            elif i == len(layers) - 1:
+                tail, pre = out_indices, head_pre
+            prelu = isinstance(act, PReLU)
+            slope = None if tail is not None else inet._slope(act, device)
+            g_z, grads[id(conv.weight)], db, dslope = spconv.wgrad(x, g, conv.weight.shape, src, pre, slope, tail,
+                                                                   slope_grad=prelu)
+            if conv.bias is not None:
+                grads[id(conv.bias)] = db
+            if prelu:
+                grads[id(act.weight)] = dslope.reshape(act.weight.shape)
+            if i > 0:  # dX: the layer on g_z with the transposed weights and the inverse rules
+                g = spconv.conv_layer(g_z, conv.weight.detach().permute(3, 1, 2, 0), None, inv, int(x.shape[0]))
+        ctx.saved = None
+        out = [grads[k].to(dt) for k, dt in zip(ctx.param_ids, ctx.param_dtypes)]
+        return (None, None, None, None, *out)
 
 
 def _check_conv(conv: SparseConv2d) -> None:

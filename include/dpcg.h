@@ -384,6 +384,47 @@ typedef struct dp_spconv_layer {
 } dp_spconv_layer_t;
 int dp_spconv_layer_f32(const dp_spconv_layer_t* layer_host, void* stream);
 
+/* ---- K6 backward: training the factor network on the device ----------------------------------------------------------
+ * Training forward: dp_spconv_layer_f32 (out bitwise the same) that also keeps what the backward reads: pre [nout,cout]
+ * = acc + bias before the activation (required when slope != NULL); with a head, hidden [nout,cout] (the activated
+ * rows the head reads) and head_pre [nout] (the head's value before the tail); with a tail and no head, head_pre [nout]
+ * (the layer's value before the tail). Pointers not required by the layer are ignored. */
+int dp_spconv_layer_train_f32(const dp_spconv_layer_t* layer_host, float* pre, float* hidden, float* head_pre,
+                              void* stream);
+/* Inverse rules: inv int32[nin, ntaps], inv[src,t] = s where rules[s,t] == src, -1 elsewhere (a tap is a fixed shift,
+ * so every slot has at most one claimant). A slot claimed twice, or a source outside [0,nin), raises DP_ERR_STRUCTURE
+ * in *flag_out. The rules of the first 2x2 layer (numbered through the sort permutation) invert in the input's order. */
+int dp_spconv_rules_invert(const int32_t* rules, int64_t nout, int32_t ntaps, int64_t nin, int32_t* inv,
+                           int32_t* flag_out, void* stream);
+/* Weight gradient of one layer, fp32 on CUDA cores, deterministic (no floating-point atomics). With x = in, g = grad_out:
+ *   grad_pre[s,co]        = g[s,co] * act'(pre[s,co])   (pre > 0 ? g : slope * g; slope == NULL: g)
+ *   grad_weight[co,t,ci]  = sum_s grad_pre[s,co] * x[src[s,t],ci]      grad_bias[co] = sum_s grad_pre[s,co]
+ *   *grad_slope           = sum over pre <= 0 of g * pre                  (optional; needs slope)
+ * tail_indices != NULL (cout == 1, slope == NULL): the output tail replaces the activation, pre = the value u before it:
+ * row < col: g * 0; row == col: u > 20 ? g : g e/(e+1), e = exp(u); else g.
+ * Sites are cut into chunks of dp_spconv_wgrad_chunk_sites(); each chunk's partial sum is one fma chain in ascending site
+ * order, the partials are added in chunk order in fp64 and rounded once: |error| <= (C + 2) 2^-24 sum|terms|, the same
+ * bits for any launch geometry. workspace: 16-byte aligned, dp_spconv_wgrad_workspace_bytes(...) bytes (0: bad shape).
+ * nout == 0 does nothing (the gradients are left as they are). The input gradient is dp_spconv_layer_f32 on grad_pre
+ * with weight'[ci,t,co] = weight[co,t,ci], src = the inverse rules, no bias and no activation. */
+typedef struct dp_spconv_grad {
+    int64_t nout;
+    int32_t ntaps, cin, cout, reserved;
+    const int32_t* src;           /* [nout, ntaps] (-1: inactive); NULL: site s reads row s (ntaps 1) */
+    const float* in;              /* [*, cin]: the layer's input */
+    const float* grad_out;        /* [nout, cout]: upstream gradient */
+    const float* pre;             /* [nout, cout] before the activation, [nout] before the tail, or NULL */
+    const float* slope;           /* device scalar or NULL: no activation */
+    const int32_t* tail_indices;  /* [nout, 3] (batch,row,col) of the output sites: the head's tail, or NULL */
+    float* grad_pre;              /* [nout, cout] */
+    float* grad_weight;           /* [cout, ntaps, cin] */
+    float* grad_bias;             /* [cout] or NULL */
+    float* grad_slope;            /* [1] or NULL */
+} dp_spconv_grad_t;
+int32_t dp_spconv_wgrad_chunk_sites(void);
+size_t dp_spconv_wgrad_workspace_bytes(int64_t nout, int32_t ntaps, int32_t cin, int32_t cout);
+int dp_spconv_wgrad_f32(const dp_spconv_grad_t* grad_host, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Diagnostics: with DPCG_TRACE=1 in the environment the fused engine records (label, clock64) pairs of CTA 0 into the
  * workspace; this copies up to `capacity` pairs to out_host[2*capacity] (label = 8*phase + point). Synchronous. */
 int dp_debug_pcg_trace(const void* workspace, int32_t nsys, int64_t* out_host, int32_t capacity);
