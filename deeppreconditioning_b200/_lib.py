@@ -77,6 +77,13 @@ class SpconvGrad(C.Structure):
                                 "grad_bias", "grad_slope")]
 
 
+class FactorSites(C.Structure):
+    """``dp_factor_sites_t``."""
+
+    _fields_ = [("nnz", _i64), ("nbatch", _i32), ("h", _i32), ("w", _i32), ("reserved", _i32)] + [
+        (name, _p) for name in ("features", "rowptr", "col", "perm", "rowptr_t", "col_t", "perm_t")]
+
+
 class DpcgError(RuntimeError):
     pass
 
@@ -132,6 +139,14 @@ _SIGNATURES = {
     "dp_spconv_wgrad_chunk_sites": (_i32, []),
     "dp_spconv_wgrad_workspace_bytes": (C.c_size_t, [_i64, _i32, _i32, _i32]),
     "dp_spconv_wgrad_f32": (C.c_int, [C.POINTER(SpconvGrad), _p, C.c_size_t, _p]),
+    "dp_sorted_spmv_f32": (C.c_int, [C.POINTER(FactorSites), _i32, _i32, _i32, _p, _p, _p]),
+    "dp_system_matvec_f32": (C.c_int, [C.POINTER(FactorSites), _i32, _i32, _p, _p, _p]),
+    "dp_llt_residual_chunk_rows": (_i32, []),
+    "dp_llt_residual_workspace_bytes": (C.c_size_t, [_i32, _i32, _i32]),
+    "dp_llt_residual_f32": (C.c_int, [C.POINTER(FactorSites), _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p, _p, _p,
+                                      C.c_size_t, _p]),
+    "dp_llt_residual_grad_f32": (C.c_int, [C.POINTER(FactorSites), _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p, _p, _p,
+                                           C.c_size_t, _p]),
     "dp_pcg_work_doubles": (_i64, [_i32]),
     "dp_pcg_workspace_bytes": (C.c_size_t, [_i32]),
     "dp_debug_pcg_trace": (C.c_int, [_p, _i32, _p, _i32]),

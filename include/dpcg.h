@@ -425,6 +425,51 @@ int32_t dp_spconv_wgrad_chunk_sites(void);
 size_t dp_spconv_wgrad_workspace_bytes(int64_t nout, int32_t ntaps, int32_t cin, int32_t cout);
 int dp_spconv_wgrad_f32(const dp_spconv_grad_t* grad_host, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- K7: deterministic training-loss products (metrics.py, utils.sparse_matvec_mul under
+ * torch.use_deterministic_algorithms) ----------------------------------------------------------------------------------
+ * The same products as dp_coo_spmv_batch_f32 in a fixed order and without floating-point atomics. A factor's sites come
+ * as two dp_spconv_sort_sites outputs: the row CSR (the call on the indices, nbatch*h rows) and the column CSR (the same
+ * call on the indices with row and column swapped, nbatch*w rows). Vectors are fp32 [nbatch, nvec, n]; sites with a row
+ * or column at or beyond n take no part (and get a zero gradient).
+ *   product   y[b,p,i] = sequential fp32 sum from 0 over row i's sites in ascending column order, every product and sum
+ *             rounded separately: bitwise dp_coo_spmv_batch_f32's oracle run on the sites sorted by (b, row, col);
+ *             the transposed product the same over the column CSR.
+ * Empty batches (nbatch, nvec or n zero) are no-ops; with zero sites the outputs are still written (zero products). */
+typedef struct dp_factor_sites {
+    int64_t nnz;              /* sites */
+    int32_t nbatch, h, w;     /* systems; spatial shape (rows, columns) */
+    int32_t reserved;
+    const float* features;    /* [nnz] in the input's site order */
+    const int32_t* rowptr; const int32_t* col; const int32_t* perm;       /* row CSR: rowptr int32[nbatch*h + 1] */
+    const int32_t* rowptr_t; const int32_t* col_t; const int32_t* perm_t; /* column CSR: rowptr_t int32[nbatch*w + 1] */
+} dp_factor_sites_t;
+/* y = T x (transpose == 0, row CSR) or T^T x (column CSR); only the CSR the product reads is required. */
+int dp_sorted_spmv_f32(const dp_factor_sites_t* sites_host, int32_t transpose, int32_t nvec, int32_t n, const float* x,
+                       float* y, void* stream);
+/* A v from the stored lower triangle T (metrics.system_matvec): y = (T v + T^T v) - D v with D v = 0 + T_ii v_i where the
+ * diagonal site is stored (0 elsewhere), each product as above. Both CSRs are required. */
+int dp_system_matvec_f32(const dp_factor_sites_t* sites_host, int32_t nvec, int32_t n, const float* v, float* y,
+                         void* stream);
+/* Loss of the form sum_p || L L^T x_p - b_p || per system (frobenius_loss, hutchinson_trace, inverse_loss):
+ *   t = L^T x, r = L t - b (fp32, kept for the backward: t, r [nbatch, nvec, n]);
+ *   S_b = sum over probes p in order of sum_i r^2, accumulated in fp64 over fixed chunks of dp_llt_residual_chunk_rows()
+ *   rows (chunks added in ascending order): the same bits for any grid, batch or site order;
+ *   terms[b] = (float) sqrt(S_b / divisor) in fp64; *loss = fp32 sum of the terms in system order (/ nbatch if mean).
+ * Both CSRs are required. workspace: 16-byte aligned, dp_llt_residual_workspace_bytes(nbatch, nvec, n) bytes (also
+ * enough for the backward). */
+int32_t dp_llt_residual_chunk_rows(void);
+size_t dp_llt_residual_workspace_bytes(int32_t nbatch, int32_t nvec, int32_t n);
+int dp_llt_residual_f32(const dp_factor_sites_t* sites_host, int32_t nvec, int32_t n, int32_t divisor, int32_t mean,
+                        const float* x, const float* b, float* t, float* r, float* terms, float* loss, void* workspace,
+                        size_t workspace_bytes, void* stream);
+/* Gradient of *loss with respect to the features of L, given the upstream gradient grad_loss (device scalar): with
+ * c_b = g' / (divisor terms[b]) (g' = grad_loss, / nbatch if mean; c_b = 0 where terms[b] == 0), rho = c_b r and
+ * s = L^T rho (a product as above), grad_features[e] for site e = (b, i, k) is sum over p in order of
+ * (rho_i t_k + x_i s_k), written in the input's site order: a closed form per site, no accumulation across sites. */
+int dp_llt_residual_grad_f32(const dp_factor_sites_t* sites_host, int32_t nvec, int32_t n, int32_t divisor, int32_t mean,
+                             const float* x, const float* t, const float* r, const float* terms, const float* grad_loss,
+                             float* grad_features, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Diagnostics: with DPCG_TRACE=1 in the environment the fused engine records (label, clock64) pairs of CTA 0 into the
  * workspace; this copies up to `capacity` pairs to out_host[2*capacity] (label = 8*phase + point). Synchronous. */
 int dp_debug_pcg_trace(const void* workspace, int32_t nsys, int64_t* out_host, int32_t capacity);
