@@ -17,6 +17,7 @@ LIB_PATH = Path(os.environ.get("DPCG_LIB") or Path(__file__).resolve().parent / 
 DP_OK = 0
 DP_ERR_STRUCTURE = 5
 DP_ERR_TIMEOUT = 6
+DP_ERR_NOT_SPD = 7
 
 PRECOND_IDENTITY, PRECOND_JACOBI, PRECOND_MULTIPLY, PRECOND_SOLVE, PRECOND_CSR = range(5)
 ENGINE_FUSED, ENGINE_STEPPED = 0, 1
@@ -147,6 +148,8 @@ _SIGNATURES = {
                                       C.c_size_t, _p]),
     "dp_llt_residual_grad_f32": (C.c_int, [C.POINTER(FactorSites), _i32, _i32, _i32, _i32, _p, _p, _p, _p, _p, _p, _p,
                                            C.c_size_t, _p]),
+    "dp_fsai_max_row_entries": (_i32, []),
+    "dp_fsai_f64": (C.c_int, [_i32, _p, _p, _p, _p, _p, _i32, _p, _p, _p]),
     "dp_pcg_work_doubles": (_i64, [_i32]),
     "dp_pcg_workspace_bytes": (C.c_size_t, [_i32]),
     "dp_debug_pcg_trace": (C.c_int, [_p, _i32, _p, _i32]),

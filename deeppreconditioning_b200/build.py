@@ -17,7 +17,7 @@ CSRC = PKG / "csrc"
 LIB_DIR = PKG / "lib"
 LIB = LIB_DIR / "libdpcg.so"
 SOURCES = ["spmv.cu", "scan.cu", "assembly.cu", "levels.cu", "sptrsv.cu", "pcg.cu", "icholt.cu", "sparseconv.cu",
-           "sparseconv_grad.cu", "losses.cu"]
+           "sparseconv_grad.cu", "losses.cu", "fsai.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17", "--fmad=false",

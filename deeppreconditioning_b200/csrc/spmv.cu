@@ -206,6 +206,7 @@ const char* dp_status_string(int status) {
         case DP_ERR_CUDA: return "CUDA runtime error";
         case DP_ERR_STRUCTURE: return "matrix structure violates the contract";
         case DP_ERR_TIMEOUT: return "dependency spin timed out";
+        case DP_ERR_NOT_SPD: return "matrix is not symmetric positive definite (non-positive pivot)";
         default: return "unknown status";
     }
 }

@@ -10,6 +10,7 @@ class                reference constructor                    apply
 ``Jacobi``           ``_construct_jacobi``    test.py:74-79   ``z = r / diag(A)``
 ``FactoredMultiply`` ``_construct_learned``   test.py:100-105 ``z = L (L^T r)``   (approximate inverse)
 ``FactoredSolve``    north_star / IC(0)                       ``z = L^-T (L^-1 r)`` (two sync-free SpTRSV)
+``fsai(A)``          no reference counterpart (comparator)    ``z = L (L^T r)``   (FSAI: a ``FactoredMultiply``)
 ``CsrOperator``      any explicit CSR ``M``   test.py:88,105  ``z = M r``
 ===================  =======================================  ==========================================
 """
@@ -401,6 +402,39 @@ def incomplete_cholesky_threshold(tril_a: CsrMatrix, fill_in: int = 1, threshold
                                   nnz.ctypes.data), "dp_icholt_host (missing diagonal or non-positive pivot)")
     k = int(nnz[0])
     return CsrMatrix.from_arrays(rowptr_out, col_out[:k].copy(), val_out[:k].copy(), device=dev)
+
+
+def fsai(A: CsrMatrix, pattern: CsrMatrix | None = None, fp32: bool = True) -> "FactoredMultiply":
+    """FSAI (factorized sparse approximate inverse, Kolotilina & Yeremin): ``M = L L^T ~ A^-1`` with ``L`` on a given
+    lower-triangular pattern, applied like the learned factor (two SpMVs, ``DP_PRECOND_MULTIPLY``).
+
+    ``A``: the full symmetric matrix. ``pattern``: lower triangular, diagonal stored, values ignored; ``tril(A)`` by
+    default. Column ``i`` of ``L`` holds ``y / sqrt(y_0)`` with ``A[J, J] y = e_0`` on the column's pattern ``J`` (at most
+    ``dp_fsai_max_row_entries()`` entries), so ``(L^T A L)_ii = 1`` (``dp_fsai_f64``). ``fp32``: every value rounded once
+    to fp32, so the factor has an exact packed copy and streams 6 bytes per entry like the learned factor; ``False``
+    keeps the fp64 values. Raises :class:`DpcgError` on a pattern the kernel does not accept and when ``A`` is not SPD."""
+    if not isinstance(A, CsrMatrix) or not isinstance(pattern, (CsrMatrix, type(None))):
+        raise _lib.DpcgError("fsai takes device CsrMatrix operands (there is no CPU path)")
+    pattern = A.tril() if pattern is None else pattern
+    if pattern.n != A.n or pattern.device != A.device:
+        raise ValueError("A and the pattern must have the same size and live on the same device")
+    lib, n, dev = _lib.lib(), A.n, A.device
+    upper = pattern.transpose()  # the pattern of U = L^T: row i is column i of L, diagonal first
+    u_val = torch.empty(max(upper.nnz, 1), dtype=torch.float64, device=dev)
+    flag = torch.zeros(1, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.dp_fsai_f64(n, _lib.ptr(A.rowptr), _lib.ptr(A.col), _lib.ptr(A.val), _lib.ptr(upper.rowptr),
+                                   _lib.ptr(upper.col), int(bool(fp32)), _lib.ptr(u_val), _lib.ptr(flag),
+                                   _lib.stream_ptr(dev)), "dp_fsai_f64")
+    status = int(flag.item())
+    if status == _lib.DP_ERR_STRUCTURE:
+        raise _lib.DpcgError(f"fsai: the pattern is not lower triangular with its diagonal in every column, a column holds "
+                             f"more than {lib.dp_fsai_max_row_entries()} entries, or A stores no diagonal in some row")
+    if status == _lib.DP_ERR_NOT_SPD:
+        raise _lib.DpcgError("fsai: A is not symmetric positive definite (non-positive pivot in a local Cholesky factor)")
+    _lib.raise_on_flag(flag, "dp_fsai_f64")
+    Lt = CsrMatrix(upper.rowptr, upper.col, u_val[: upper.nnz], n)
+    return FactoredMultiply(Lt.transpose(), Lt)
 
 
 class _Operator:

@@ -31,7 +31,7 @@ import torch
 from . import _lib
 from .cg import PcgBatch
 from .distributed import gather_records, shard_indices
-from .precond import (CsrOperator, FactoredMultiply, FactoredSolve, Identity, Jacobi, incomplete_cholesky0,
+from .precond import (CsrOperator, FactoredMultiply, FactoredSolve, Identity, Jacobi, fsai, incomplete_cholesky0,
                       incomplete_cholesky_threshold, level_ordering)
 from .sparse import CsrMatrix
 
@@ -54,6 +54,10 @@ class BenchmarkSuite:
         ic_apply: how the incomplete-Cholesky comparator is applied: ``"solve"`` (two triangular solves, ``z = L^-T L^-1 r``,
             what an IC preconditioner is) or ``"multiply"`` (the reference's literal ``(L L^T) @ r``, ``test.py:88``, which
             its authors tag "unstable", ``test.py:45``; SURVEY D2).
+
+    Two techniques beyond the reference can be named in ``techniques``: ``"fsai"`` (FSAI on the pattern of ``tril(A)``)
+    and ``"fsai_learned"`` (FSAI on the pattern of the learned factor, whose set-up time includes the model forward that
+    supplies the pattern). Both are approximate-inverse factors applied like the learned one, two SpMVs per iteration.
     """
 
     data_set: object
@@ -123,6 +127,20 @@ class BenchmarkSuite:
         lower_t = CsrMatrix.from_spconv(preconditioners_tril, original_size, mode="tril_t")
         return FactoredMultiply(lower, lower_t)
 
+    def _construct_fsai(self, matrix: CsrMatrix):
+        """FSAI on the pattern of ``tril(A)`` (``precond.fsai``): the classical factor of the learned factor's kind."""
+        self.variants["fsai"] = "FSAI on tril(A) (GPU), fp32 values, applied by multiply"
+        return fsai(matrix, self._tril_of(matrix))
+
+    def _construct_fsai_learned(self, system_tril, original_size: int):
+        """FSAI on the pattern of the ``L`` that ``_construct_learned`` assembles: the classical factor that streams the
+        same bytes per iteration as the learned one. Its set-up time covers the model forward that supplies the pattern
+        and the assembly of ``A`` from ``system_tril`` besides the FSAI kernel."""
+        pattern = self._construct_learned(system_tril, original_size).L
+        matrix = CsrMatrix.from_spconv(system_tril, original_size, mode="symmetrise")
+        self.variants["fsai_learned"] = "FSAI on the pattern of the learned L (GPU), fp32 values, applied by multiply"
+        return fsai(matrix, pattern)
+
     def _tril_of(self, matrix: CsrMatrix) -> CsrMatrix:
         lower = getattr(matrix, "_lower", None)
         return lower if lower is not None else matrix.tril()
@@ -178,8 +196,8 @@ class BenchmarkSuite:
                 for system_tril, matrix, rhs, n in prepared:
                     torch.cuda.synchronize()
                     start_time = time.perf_counter()
-                    if name == "learned":
-                        preconditioner = self._construct_learned(system_tril, n)
+                    if name in ("learned", "fsai_learned"):
+                        preconditioner = getattr(self, f"_construct_{name}")(system_tril, n)
                     elif name == "incomplete_cholesky":
                         preconditioner = self._construct_incomplete_cholesky(matrix, self.ic_fill_in, self.ic_threshold)
                     else:

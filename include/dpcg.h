@@ -33,7 +33,8 @@ enum dp_status {
     DP_ERR_WORKSPACE = 3,  /* workspace too small */
     DP_ERR_CUDA = 4,       /* a CUDA runtime call failed; see dp_last_cuda_error() */
     DP_ERR_STRUCTURE = 5,  /* matrix structure violates the contract (reported through a device flag, see below) */
-    DP_ERR_TIMEOUT = 6     /* a dependency spin exceeded its budget (device flag) */
+    DP_ERR_TIMEOUT = 6,    /* a dependency spin exceeded its budget (device flag) */
+    DP_ERR_NOT_SPD = 7     /* a Cholesky pivot was not positive: the matrix is not SPD (device flag) */
 };
 
 /* Preconditioner application z = M r inside the loop (reference: `zk = M @ rk`, cg.py:61,81). */
@@ -469,6 +470,24 @@ int dp_llt_residual_f32(const dp_factor_sites_t* sites_host, int32_t nvec, int32
 int dp_llt_residual_grad_f32(const dp_factor_sites_t* sites_host, int32_t nvec, int32_t n, int32_t divisor, int32_t mean,
                              const float* x, const float* t, const float* r, const float* terms, const float* grad_loss,
                              float* grad_features, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- K8: FSAI factor on a given pattern (the classical approximate-inverse comparator of the learned factor) ------------
+ * Factorized sparse approximate inverse (Kolotilina & Yeremin): M = L L^T ~ A^-1 with L lower triangular on a fixed
+ * pattern, applied like the learned factor (DP_PRECOND_MULTIPLY). The call fills U = L^T: u_rowptr / u_col is the CSR of
+ * U (the transpose of L's pattern, dp_csr_transpose), and row i of U, pattern J = (j_0 = i < j_1 < ... < j_{k-1}),
+ * gets y_p / sqrt(y_0) where A[J, J] y = e_0, so that (L^T A L)_ii = 1. A is the full symmetric CSR (sorted rows);
+ * entries of A[J, J] it does not store are 0. Fixed arithmetic order, every operation rounded separately: the Cholesky
+ * factor R of A[J, J] left-looking by columns, forward then backward substitution, each sum subtracted term by term in
+ * ascending index (csrc/fsai.cu): the same bits as oracle_fsai. fp32 == 1 rounds every value once to fp32 (widened back
+ * to fp64 in u_val), so the factor has an exact packed copy (dp_csr_pack). u_val has room for nnz(U) doubles.
+ * *flag_out (device int32): DP_ERR_STRUCTURE for a row of U that does not start with its diagonal, has columns that do
+ * not ascend or lie outside [0, n), or has more than dp_fsai_max_row_entries() entries, or a diagonal entry A does not
+ * store; DP_ERR_NOT_SPD for a pivot that is not positive (or NaN). The values of a flagged row are not written.
+ * n == 0 does nothing. One warp per row: rows of up to 32 entries (the factor network's pattern holds at most 15 per
+ * column on 2-D and 24 on 3-D 7-point systems). */
+int32_t dp_fsai_max_row_entries(void);
+int dp_fsai_f64(int32_t n, const int32_t* a_rowptr, const int32_t* a_col, const double* a_val, const int32_t* u_rowptr,
+                const int32_t* u_col, int32_t fp32, double* u_val, int32_t* flag_out, void* stream);
 
 /* Diagnostics: with DPCG_TRACE=1 in the environment the fused engine records (label, clock64) pairs of CTA 0 into the
  * workspace; this copies up to `capacity` pairs to out_host[2*capacity] (label = 8*phase + point). Synchronous. */
