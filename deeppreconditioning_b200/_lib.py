@@ -100,6 +100,9 @@ _SIGNATURES = {
     "dp_csr_transpose": (C.c_int, [_i32, _i32, _p, _p, _p, _p, _p, _p, _p, C.c_size_t, _p]),
     "dp_csr_inv_diagonal": (C.c_int, [_i32, _p, _p, _p, _p, _p, _p]),
     "dp_csr_aat_nnz": (C.c_int, [_i32, _p, _p, _p, _p, _p, _p]),
+    "dp_csr_pattern_product_workspace_bytes": (C.c_size_t, [_i32]),
+    "dp_csr_pattern_product_count": (C.c_int, [_i32, _p, _p, _p, _p, _i32, _p, _p, _p, _p, C.c_size_t, _p]),
+    "dp_csr_pattern_product_fill": (C.c_int, [_i32, _p, _p, _p, _p, _i32, _p, _p, _p]),
     "dp_spmv_csr_f64": (C.c_int, [_i32, _i32, _p, _p, _p, _p, _p, _p]),
     "dp_csr_pack_tile_rows": (_i32, []),
     "dp_csr_pack": (C.c_int, [_i32, _i32, _p, _p, _p, _p, _p, _p, _p, _p]),

@@ -7,6 +7,8 @@
 //   fill   : entries dropped into their row segment at an atomically claimed slot (order inside a row arbitrary)
 //   sort   : every row sorted by column -> the output no longer depends on the atomic order: bit-exact
 //            against torch's to_sparse_csr() / scipy; a repeated (row, col) raises DP_ERR_STRUCTURE.
+// Symbolic product of two patterns (FSAI power patterns, the density count): count rows, scan, fill first occurrences,
+// sort rows - the same integer pipeline with the row union (row_union) as the count and the fill.
 #include "common.cuh"
 #include "scan.cuh"
 
@@ -70,24 +72,26 @@ __global__ void coo_fill_kernel(const int* __restrict__ ind, const float* __rest
 }
 
 // One thread per row: insertion sort by column (rows on this path hold 3..~25 entries), then duplicate check.
+// val == NULL: a pattern without values; flag == NULL: no duplicate check.
 __global__ void csr_sort_rows_kernel(int n, const int* __restrict__ rowptr, int* __restrict__ col,
                                      double* __restrict__ val, int* __restrict__ flag) {
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         const int rs = rowptr[i], re = rowptr[i + 1];
         for (int p = rs + 1; p < re; ++p) {
             const int kc = col[p];
-            const double kv = val[p];
+            const double kv = val ? val[p] : 0.0;
             int q = p - 1;
             while (q >= rs && col[q] > kc) {
                 col[q + 1] = col[q];
-                val[q + 1] = val[q];
+                if (val) val[q + 1] = val[q];
                 --q;
             }
             col[q + 1] = kc;
-            val[q + 1] = kv;
+            if (val) val[q + 1] = kv;
         }
-        for (int p = rs + 1; p < re; ++p)
-            if (col[p] == col[p - 1]) atomicCAS(flag, 0, (int)DP_ERR_STRUCTURE);
+        if (flag)
+            for (int p = rs + 1; p < re; ++p)
+                if (col[p] == col[p - 1]) atomicCAS(flag, 0, (int)DP_ERR_STRUCTURE);
     }
 }
 
@@ -130,42 +134,88 @@ __global__ void inv_diagonal_kernel(int n, const int* __restrict__ rowptr, const
 }
 
 
-// nnz(L L^T) without forming the product (test.py:107-109 reports the density of the explicit M = L L^T that
-// test.py:104-105 stores): entry (i, j) is structurally non-zero iff rows i and j of L share a column, i.e.
-//   row i of L L^T  =  union over the columns c of row i of { rows j with L_jc != 0 }  =  union of rows c of L^T.
-// One warp per row: candidate j from the k-th list counts iff it is in none of the lists 0..k-1 (binary search, every
-// row of L^T is sorted). Integer work, exact; a 64-bit total by atomics.
-__global__ void __launch_bounds__(256) aat_nnz_kernel(int n, const int* __restrict__ rowptr, const int* __restrict__ col,
-                                                      const int* __restrict__ rowptr_t, const int* __restrict__ col_t,
-                                                      unsigned long long* __restrict__ total) {
+// Row i of the structural product C = P Q (values never read, nothing cancels): the union, over the columns c of row i
+// of P, of row c of Q. One warp per row; the lanes take the entries of row c of Q 32 at a time, and candidate j is a
+// FIRST occurrence iff it lies in none of the rows c' of Q for the columns c' before c in row i of P (binary search:
+// every row of Q is sorted). No buffer, so no cap on the length of a row of C. lower: candidates j > i take no part.
+// Columns of P or Q outside [0, n) are skipped and raise DP_ERR_STRUCTURE in *flag (when flag != NULL).
+// emit(first, j) is called by all 32 lanes together, once per group of 32 candidates and in candidate order (lanes past
+// the end of the row of Q pass first = false), so a caller can count by ballot or place first occurrences by prefix.
+template <class Emit>
+__device__ __forceinline__ void row_union(int i, int n, const int* __restrict__ p_rowptr, const int* __restrict__ p_col,
+                                          const int* __restrict__ q_rowptr, const int* __restrict__ q_col, int lower,
+                                          int* __restrict__ flag, Emit&& emit) {
+    const int lane = threadIdx.x & 31;
+    const int rs = p_rowptr[i], re = p_rowptr[i + 1];
+    for (int k = rs; k < re; ++k) {
+        const int c = p_col[k];
+        if ((unsigned)c >= (unsigned)n) {
+            if (flag && lane == 0) atomicCAS(flag, 0, (int)DP_ERR_STRUCTURE);
+            continue;
+        }
+        const int ts = q_rowptr[c], te = q_rowptr[c + 1];
+        for (int base = ts; base < te; base += 32) {
+            const int q = base + lane;
+            const int j = q < te ? q_col[q] : -1;
+            bool first = false;
+            if (q < te && (unsigned)j >= (unsigned)n) {
+                if (flag) atomicCAS(flag, 0, (int)DP_ERR_STRUCTURE);
+            } else if (q < te && (!lower || j <= i)) {
+                first = true;
+                for (int k2 = rs; k2 < k && first; ++k2) {
+                    const int c2 = p_col[k2];
+                    if ((unsigned)c2 >= (unsigned)n) continue;
+                    int lo = q_rowptr[c2], hi = q_rowptr[c2 + 1];
+                    while (lo < hi) {
+                        const int mid = (lo + hi) >> 1;
+                        const int v = q_col[mid];
+                        if (v == j) { first = false; break; }
+                        if (v < j) lo = mid + 1; else hi = mid;
+                    }
+                }
+            }
+            emit(first, j);
+        }
+    }
+}
+
+// Entries per row of C = P Q (counts[i], when counts != NULL) and their 64-bit total by atomics. Integer work, exact.
+// Also the count behind dp_csr_aat_nnz: nnz(L L^T) without forming the product (test.py:107-109 reports the density of
+// the explicit M = L L^T that test.py:104-105 stores) is this count with P = L, Q = L^T.
+__global__ void __launch_bounds__(256) pattern_count_kernel(int n, const int* __restrict__ p_rowptr,
+                                                            const int* __restrict__ p_col, const int* __restrict__ q_rowptr,
+                                                            const int* __restrict__ q_col, int lower,
+                                                            int* __restrict__ counts, unsigned long long* __restrict__ total,
+                                                            int* __restrict__ flag) {
     const int lane = threadIdx.x & 31;
     const int warps = (gridDim.x * blockDim.x) >> 5;
     unsigned long long mine = 0;
     for (int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += warps) {
-        const int rs = rowptr[i], re = rowptr[i + 1];
-        for (int k = rs; k < re; ++k) {
-            const int c = col[k];
-            const int ts = rowptr_t[c], te = rowptr_t[c + 1];
-            for (int q = ts + lane; q < te; q += 32) {
-                const int j = col_t[q];
-                bool seen = false;
-                for (int k2 = rs; k2 < k && !seen; ++k2) {
-                    const int c2 = col[k2];
-                    int lo = rowptr_t[c2], hi = rowptr_t[c2 + 1];
-                    while (lo < hi) {
-                        const int mid = (lo + hi) >> 1;
-                        const int v = col_t[mid];
-                        if (v == j) { seen = true; break; }
-                        if (v < j) lo = mid + 1; else hi = mid;
-                    }
-                }
-                mine += seen ? 0ull : 1ull;
-            }
-        }
+        int row = 0;
+        row_union(i, n, p_rowptr, p_col, q_rowptr, q_col, lower, flag,
+                  [&](bool first, int) { row += __popc(__ballot_sync(kFull, first)); });
+        if (counts && lane == 0) counts[i] = row;
+        mine += (unsigned long long)row;
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) mine += __shfl_xor_sync(kFull, mine, o);
     if (lane == 0 && mine) atomicAdd(total, mine);
+}
+
+// Row i of C written at c_rowptr[i] in candidate order (first occurrences only, placed by a warp prefix of the ballot):
+// the same entries pattern_count_kernel counted, deterministic, sorted afterwards by csr_sort_rows_kernel.
+__global__ void __launch_bounds__(256) pattern_fill_kernel(int n, const int* __restrict__ p_rowptr,
+                                                           const int* __restrict__ p_col, const int* __restrict__ q_rowptr,
+                                                           const int* __restrict__ q_col, int lower,
+                                                           const int* __restrict__ c_rowptr, int* __restrict__ c_col) {
+    const int lane = threadIdx.x & 31;
+    const int warps = (gridDim.x * blockDim.x) >> 5;
+    for (int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += warps) {
+        int pos = c_rowptr[i];
+        row_union(i, n, p_rowptr, p_col, q_rowptr, q_col, lower, nullptr, [&](bool first, int j) {
+            const unsigned mask = __ballot_sync(kFull, first);
+            if (first) c_col[pos + __popc(mask & ((1u << lane) - 1u))] = j;
+            pos += __popc(mask);
+        });
+    }
 }
 
 static int grid_for(long long items, int threads) {
@@ -271,8 +321,49 @@ int dp_csr_aat_nnz(int32_t n, const int32_t* rowptr, const int32_t* col, const i
     cudaStream_t s = (cudaStream_t)stream;
     DP_CUDA(cudaMemsetAsync(nnz_out, 0, sizeof(int64_t), s));
     if (n == 0) return DP_OK;
-    aat_nnz_kernel<<<grid_for((long long)n * 32, 256), 256, 0, s>>>(n, rowptr, col, rowptr_t, col_t,
-                                                                    reinterpret_cast<unsigned long long*>(nnz_out));
+    pattern_count_kernel<<<grid_for((long long)n * 32, 256), 256, 0, s>>>(
+        n, rowptr, col, rowptr_t, col_t, 0, nullptr, reinterpret_cast<unsigned long long*>(nnz_out), nullptr);
+    DP_LAUNCH_CHECK();
+    return DP_OK;
+}
+
+size_t dp_csr_pattern_product_workspace_bytes(int32_t n) { return scan_workspace_bytes((long long)(n < 0 ? 0 : n) + 1); }
+
+int dp_csr_pattern_product_count(int32_t n, const int32_t* p_rowptr, const int32_t* p_col, const int32_t* q_rowptr,
+                                 const int32_t* q_col, int32_t lower, int32_t* c_rowptr, int64_t* nnz_out,
+                                 int32_t* flag_out, void* workspace, size_t workspace_bytes, void* stream) {
+    if (n < 0 || (lower != 0 && lower != 1)) return DP_ERR_INVALID;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (n == 0) {  // the empty product: rowptr = {0}, total 0 (outputs that are not given are left alone)
+        if (c_rowptr) DP_CUDA(cudaMemsetAsync(c_rowptr, 0, sizeof(int32_t), s));
+        if (nnz_out) DP_CUDA(cudaMemsetAsync(nnz_out, 0, sizeof(int64_t), s));
+        return DP_OK;
+    }
+    if (!p_rowptr || !p_col || !q_rowptr || !q_col || !c_rowptr || !nnz_out || !flag_out || !workspace)
+        return DP_ERR_INVALID;
+    if (!aligned16(workspace)) return DP_ERR_ALIGNMENT;
+    if (workspace_bytes < dp_csr_pattern_product_workspace_bytes(n)) return DP_ERR_WORKSPACE;
+    DP_CUDA(cudaMemsetAsync(nnz_out, 0, sizeof(int64_t), s));
+    DP_CUDA(cudaMemsetAsync(c_rowptr + n, 0, sizeof(int32_t), s));
+    // row counts land in c_rowptr[0..n) and are scanned in place into the row pointers
+    pattern_count_kernel<<<grid_for((long long)n * 32, 256), 256, 0, s>>>(
+        n, p_rowptr, p_col, q_rowptr, q_col, lower, c_rowptr, reinterpret_cast<unsigned long long*>(nnz_out), flag_out);
+    DP_LAUNCH_CHECK();
+    return exclusive_scan_i32(c_rowptr, c_rowptr, (long long)n + 1, workspace, s);
+}
+
+int dp_csr_pattern_product_fill(int32_t n, const int32_t* p_rowptr, const int32_t* p_col, const int32_t* q_rowptr,
+                                const int32_t* q_col, int32_t lower, const int32_t* c_rowptr, int32_t* c_col,
+                                void* stream) {
+    if (n < 0 || (lower != 0 && lower != 1)) return DP_ERR_INVALID;
+    if (n == 0) return DP_OK;
+    if (!p_rowptr || !p_col || !q_rowptr || !q_col || !c_rowptr || !c_col) return DP_ERR_INVALID;
+    if (!aligned16(c_col)) return DP_ERR_ALIGNMENT;
+    cudaStream_t s = (cudaStream_t)stream;
+    pattern_fill_kernel<<<grid_for((long long)n * 32, 256), 256, 0, s>>>(n, p_rowptr, p_col, q_rowptr, q_col, lower,
+                                                                         c_rowptr, c_col);
+    DP_LAUNCH_CHECK();
+    csr_sort_rows_kernel<<<grid_for(n, 128), 128, 0, s>>>(n, c_rowptr, c_col, nullptr, nullptr);
     DP_LAUNCH_CHECK();
     return DP_OK;
 }

@@ -10,7 +10,8 @@ class                reference constructor                    apply
 ``Jacobi``           ``_construct_jacobi``    test.py:74-79   ``z = r / diag(A)``
 ``FactoredMultiply`` ``_construct_learned``   test.py:100-105 ``z = L (L^T r)``   (approximate inverse)
 ``FactoredSolve``    north_star / IC(0)                       ``z = L^-T (L^-1 r)`` (two sync-free SpTRSV)
-``fsai(A)``          no reference counterpart (comparator)    ``z = L (L^T r)``   (FSAI: a ``FactoredMultiply``)
+``fsai(A)``          no reference counterpart (comparator)    ``z = L (L^T r)``   (FSAI: a ``FactoredMultiply``; its
+                                                              patterns: ``tril(A)``, ``power_pattern(A, k)``, any)
 ``CsrOperator``      any explicit CSR ``M``   test.py:88,105  ``z = M r``
 ===================  =======================================  ==========================================
 """
@@ -435,6 +436,58 @@ def fsai(A: CsrMatrix, pattern: CsrMatrix | None = None, fp32: bool = True) -> "
     _lib.raise_on_flag(flag, "dp_fsai_f64")
     Lt = CsrMatrix(upper.rowptr, upper.col, u_val[: upper.nnz], n)
     return FactoredMultiply(Lt.transpose(), Lt)
+
+
+_INT32_MAX = 2**31 - 1
+
+
+def _pattern_product(P: CsrMatrix, Q: CsrMatrix, lower: bool) -> CsrMatrix:
+    """The structural pattern of ``P Q`` (``tril`` of it with ``lower``), every value 1.0: ``dp_csr_pattern_product_count``,
+    one read-back of the total and the device flag, then ``dp_csr_pattern_product_fill``."""
+    lib, n, dev = _lib.lib(), P.n, P.device
+    if Q.n != n or Q.device != dev:
+        raise ValueError("P and Q must have the same size and live on the same device")
+    rowptr = torch.empty(n + 1, dtype=torch.int32, device=dev)
+    total = torch.zeros(1, dtype=torch.int64, device=dev)
+    flag = torch.zeros(1, dtype=torch.int32, device=dev)
+    ws = _workspace(lib.dp_csr_pattern_product_workspace_bytes(n), dev)
+    operands = (_lib.ptr(P.rowptr), _lib.ptr(P.col), _lib.ptr(Q.rowptr), _lib.ptr(Q.col), int(bool(lower)))
+    with torch.cuda.device(dev):
+        _lib.check(lib.dp_csr_pattern_product_count(n, *operands, _lib.ptr(rowptr), _lib.ptr(total), _lib.ptr(flag),
+                                                     _lib.ptr(ws), ws.numel(), _lib.stream_ptr(dev)),
+                   "dp_csr_pattern_product_count")
+    nnz, status = torch.cat([total, flag.to(torch.int64)]).tolist()
+    if status:
+        raise _lib.DpcgError(f"pattern product: a column index lies outside [0, {n})")
+    if nnz > _INT32_MAX:
+        raise _lib.DpcgError(f"pattern product: the result holds {nnz} entries, more than an int32 CSR can index "
+                             f"({_INT32_MAX})")
+    col = torch.empty(max(nnz, 1), dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.dp_csr_pattern_product_fill(n, *operands, _lib.ptr(rowptr), _lib.ptr(col), _lib.stream_ptr(dev)),
+                   "dp_csr_pattern_product_fill")
+    return CsrMatrix(rowptr, col[:nnz], torch.ones(nnz, dtype=torch.float64, device=dev), n)
+
+
+def power_pattern(A: CsrMatrix, power: int = 2) -> CsrMatrix:
+    """The pattern of ``tril(|A|^power)``, every value 1.0: the standard a priori FSAI patterns (Chow, 2000), for
+    ``fsai(A, power_pattern(A, k))``. Built on the device by symbolic products (``dp_csr_pattern_product_*``): ``A``,
+    then ``power - 2`` full products with ``A``, then one that keeps the lower triangle. ``power = 1`` is the structure
+    of ``A.tril()``. Columns grow with ``power``: at most ``k² + k + 1`` entries on a 2-D 5-point system (3, 7, 13, 21, 31
+    for k = 1…5) and 4, 13, 32, 65 on a 3-D 7-point one, and ``fsai`` takes columns of at most
+    ``dp_fsai_max_row_entries()`` = 32 entries. Raises :class:`DpcgError` for CPU operands and when a product
+    would hold more than ``2^31 - 1`` entries, ``ValueError`` for a power that is not an integer of at least 1."""
+    if isinstance(power, bool) or not isinstance(power, (int, np.integer)) or power < 1:
+        raise ValueError(f"power_pattern: power must be an integer >= 1, got {power!r}")
+    if not isinstance(A, CsrMatrix):
+        raise _lib.DpcgError("power_pattern takes a device CsrMatrix (there is no CPU path)")
+    if power == 1:
+        lower = A.tril()
+        return CsrMatrix(lower.rowptr, lower.col, torch.ones(lower.nnz, dtype=torch.float64, device=A.device), A.n)
+    P = A
+    for _ in range(int(power) - 2):
+        P = _pattern_product(P, A, lower=False)
+    return _pattern_product(P, A, lower=True)
 
 
 class _Operator:

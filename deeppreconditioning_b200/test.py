@@ -32,7 +32,7 @@ from . import _lib
 from .cg import PcgBatch
 from .distributed import gather_records, shard_indices
 from .precond import (CsrOperator, FactoredMultiply, FactoredSolve, Identity, Jacobi, fsai, incomplete_cholesky0,
-                      incomplete_cholesky_threshold, level_ordering)
+                      incomplete_cholesky_threshold, level_ordering, power_pattern)
 from .sparse import CsrMatrix
 
 RESULTS_DIRECTORY: Path = Path("./assets/results/")
@@ -55,9 +55,10 @@ class BenchmarkSuite:
             what an IC preconditioner is) or ``"multiply"`` (the reference's literal ``(L L^T) @ r``, ``test.py:88``, which
             its authors tag "unstable", ``test.py:45``; SURVEY D2).
 
-    Two techniques beyond the reference can be named in ``techniques``: ``"fsai"`` (FSAI on the pattern of ``tril(A)``)
+    Three techniques beyond the reference can be named in ``techniques``: ``"fsai"`` (FSAI on the pattern of ``tril(A)``),
+    ``"fsai_power"`` (FSAI on the pattern of ``tril(|A|^fsai_power)``, whose set-up time includes building that pattern)
     and ``"fsai_learned"`` (FSAI on the pattern of the learned factor, whose set-up time includes the model forward that
-    supplies the pattern). Both are approximate-inverse factors applied like the learned one, two SpMVs per iteration.
+    supplies the pattern). All are approximate-inverse factors applied like the learned one, two SpMVs per iteration.
     """
 
     data_set: object
@@ -71,6 +72,7 @@ class BenchmarkSuite:
     ic_apply: str = "solve"
     ic_fill_in: int = 1        # the arguments run() hands to _construct_incomplete_cholesky: the reference's defaults
     ic_threshold: float = 0.1  # (test.py:81); (0, 0.0) selects IC(0) on the GPU
+    fsai_power: int = 2        # "fsai_power": FSAI on tril(|A|^fsai_power)
     kappas: dict = field(default_factory=dict)
     densities: dict = field(default_factory=dict)
     iterations: dict = field(default_factory=dict)
@@ -131,6 +133,11 @@ class BenchmarkSuite:
         """FSAI on the pattern of ``tril(A)`` (``precond.fsai``): the classical factor of the learned factor's kind."""
         self.variants["fsai"] = "FSAI on tril(A) (GPU), fp32 values, applied by multiply"
         return fsai(matrix, self._tril_of(matrix))
+
+    def _construct_fsai_power(self, matrix: CsrMatrix):
+        """FSAI on the pattern of ``tril(|A|^fsai_power)`` (``precond.power_pattern``, built on the device)."""
+        self.variants["fsai_power"] = f"FSAI on tril(|A|^{self.fsai_power}) (GPU), fp32 values, applied by multiply"
+        return fsai(matrix, power_pattern(matrix, self.fsai_power))
 
     def _construct_fsai_learned(self, system_tril, original_size: int):
         """FSAI on the pattern of the ``L`` that ``_construct_learned`` assembles: the classical factor that streams the

@@ -92,6 +92,24 @@ int dp_csr_inv_diagonal(int32_t n, const int32_t* rowptr, const int32_t* col, co
 int dp_csr_aat_nnz(int32_t n, const int32_t* rowptr, const int32_t* col, const int32_t* rowptr_t, const int32_t* col_t,
                    int64_t* nnz_out, void* stream);
 
+/* Symbolic sparse product: C = the structural pattern of P Q for n x n patterns P and Q (CSR; rows of Q sorted, no
+ * repeats). Values are never read, so nothing cancels: row i of C is the union, over the columns c of row i of P, of
+ * row c of Q; with lower == 1 entries with column > i are dropped (tril). dp_csr_aat_nnz is this count with P = L, Q = L^T. Two steps,
+ * because the caller sizes the output:
+ *   _count writes c_rowptr int32[n+1] and *nnz_out (DEVICE int64, the total); c_rowptr is valid only when the total is at
+ *          most INT32_MAX, which the caller checks before _fill. *flag_out (device int32) receives DP_ERR_STRUCTURE for a
+ *          column of P or Q outside [0, n). workspace: 16-byte aligned, dp_csr_pattern_product_workspace_bytes(n) bytes.
+ *          n == 0 writes c_rowptr[0] = 0 and a total of 0 (each when given) and needs nothing else.
+ *   _fill  writes c_col int32[total] (16-byte aligned): every row sorted ascending, no duplicates.
+ * No cap on the length of a row. Exact integer work, the same output for any launch geometry. */
+size_t dp_csr_pattern_product_workspace_bytes(int32_t n);
+int dp_csr_pattern_product_count(int32_t n, const int32_t* p_rowptr, const int32_t* p_col, const int32_t* q_rowptr,
+                                 const int32_t* q_col, int32_t lower, int32_t* c_rowptr, int64_t* nnz_out,
+                                 int32_t* flag_out, void* workspace, size_t workspace_bytes, void* stream);
+int dp_csr_pattern_product_fill(int32_t n, const int32_t* p_rowptr, const int32_t* p_col, const int32_t* q_rowptr,
+                                const int32_t* q_col, int32_t lower, const int32_t* c_rowptr, int32_t* c_col,
+                                void* stream);
+
 /* ---- packed stream copy of a CSR matrix (lossless) -----------------------------------------------------------
  * The operands of this path are fp32 data widened to fp64 (the CNN output and the data set's matrices are fp32,
  * test.py:100-105, data_set.py:121-125) on banded patterns, so the 12 bytes per stored entry of the fp64/int32 CSR

@@ -7,11 +7,13 @@ repetitions (mean and min per call):
   fsai_kernel_*       dp_fsai_f64 alone on the pattern of U = L^T made beforehand, per pattern (tril(A), learned L);
   fsai_*              precond.fsai(A, pattern): the transpose of the pattern, the kernel, the transpose of U, and the
                       packed copies of L and L^T (dp_csr_pack) that the fused PCG engine streams;
-  learned             InferenceNet forward on the batch and the L / L^T assembly (CsrMatrix.from_spconv) of every system.
+  learned             InferenceNet forward on the batch and the L / L^T assembly (CsrMatrix.from_spconv) of every system;
+  power_pattern_k     precond.power_pattern(A, k) alone: the pattern of tril(|A|^k) by symbolic products, k = 2, 3, 4;
+  fsai_power_k        power_pattern(A, k) and precond.fsai on it, with the packed copies of L and L^T.
 FSAI has no batched entry point: 8 systems are 8 calls in a row (one system has ~10^5 independent rows).
 Solve: one PcgBatch of --systems systems of the bench set (systems 0.., seeds of synthetic.poisson2d_tril), rtol 1e-8 on
 the squared criterion, max_iter 20000, fused engine on the packed copies, per technique learned / fsai_learned / fsai /
-jacobi: iterations (mean, min, max) and the time of one solve (CUDA events, after one warm-up solve).
+fsai_power_2..4 / jacobi: iterations (mean, min, max) and the time of one solve (CUDA events, after one warm-up solve).
 Prints one JSON line with the GPU's name and power limit read in the same run (and writes it to DIR/fsai_bench.json).
 """
 from __future__ import annotations
@@ -35,6 +37,7 @@ from inference_bench import gpu_info, timed  # noqa: E402
 
 CNN_BATCH = 8
 RTOL, MAX_ITER = 1e-8, 20000
+POWERS = (2, 3, 4)
 
 
 def make_systems(indices, side, inet, device):
@@ -84,6 +87,18 @@ def setup_case(systems, inet, side, reps) -> dict:
         res[f"fsai_{name}"] = timed(full, reps)
         res[f"nnz_per_row_{name}"] = sum(u.nnz for u in uppers) / sum(u.n for u in uppers)
         res[f"longest_column_{name}"] = max(int(torch.diff(u.rowptr).max()) for u in uppers)
+    for k in POWERS:
+        res[f"power_pattern_{k}"] = timed(lambda: [precond.power_pattern(A, k) for A, _, _ in systems], reps)
+
+        def full_power():
+            ops = [precond.fsai(A, precond.power_pattern(A, k)) for A, _, _ in systems]
+            pack_many([m for op in ops for m in (op.L, op.Lt)])
+            return ops
+
+        res[f"fsai_power_{k}"] = timed(full_power, reps)
+        uppers = [precond.power_pattern(A, k).transpose() for A, _, _ in systems]
+        res[f"nnz_per_row_power_{k}"] = sum(u.nnz for u in uppers) / sum(u.n for u in uppers)
+        res[f"longest_column_power_{k}"] = max(int(torch.diff(u.rowptr).max()) for u in uppers)
     st, _, _, sizes = synthetic.make_batch("poisson2d", side, list(range(nsys)), device=device)
 
     def learned():
@@ -100,6 +115,7 @@ def solve_case(systems) -> dict:
     ops = {"learned": lambda A, M: M,
            "fsai_learned": lambda A, M: precond.fsai(A, M.L),
            "fsai": lambda A, M: precond.fsai(A),
+           **{f"fsai_power_{k}": (lambda k: lambda A, M: precond.fsai(A, precond.power_pattern(A, k)))(k) for k in POWERS},
            "jacobi": lambda A, M: dp.Jacobi(A)}
     res = {}
     for name, make in ops.items():
